@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — DSAC-T gradient-steps/sec on synthetic Humanoid-shaped minibatches.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 4096]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 4096] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): obs=376, act=17, MLP [256,256,256] for the policy and both
 critics, batch 4096 per GPU, device replay ring of 1e6 synthetic transitions (3.09 GB, far larger
@@ -58,7 +58,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dp", default="peer", choices=["peer", "nccl"],
                     help="N > 1: exchanges inside the step's kernels over NVLink peer memory, or torch.distributed/NCCL")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed (the networks' weights under their "
+                         "state_dict names, and tb_info.npy) to DIR/<name>.npy, so that two builds run with the same "
+                         "arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def peaks():
@@ -307,6 +314,18 @@ def check_replicas(alg, eng, cfg, B, rank, world, dev, dist, it0):
     return out
 
 
+def dump_outputs(eng, out_dir, global_batch):
+    """What a caller of the timed update holds after its last step: every network's parameters and target parameters
+    under their state_dict names (float32), and `tb_info.npy`, the 14 tb_info values in engine.STAT_KEYS order (float64).
+    About 5.6 MB for the Humanoid networks."""
+    from dsac_v2_b200.engine import STAT_KEYS
+    os.makedirs(out_dir, exist_ok=True)
+    stats = eng.read_stats(global_batch)
+    np.save(os.path.join(out_dir, "tb_info.npy"), np.array([stats[k] for k in STAT_KEYS], dtype=np.float64))
+    for name, t in eng.export_weights().items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy().astype(np.float32))
+
+
 def _lib_mode(eng):
     from dsac_v2_b200 import _lib
     return {v: k for k, v in _lib.GEMM_MODES.items()}[eng.cfg.gemm_mode]
@@ -441,6 +460,8 @@ def main():
             dev_step(it); it += 1
         e1.record()
         barrier()
+        if args.dump_outputs and rank == 0:   # before the sampler's extra steps below, whose count depends on timing
+            dump_outputs(eng, args.dump_outputs, B * world)
         extra = max(0.0, 1.2 - e0.elapsed_time(e1) / 1000)  # keep the sampler alive for a few readings
         n_extra = torch.tensor([int(extra * 1000 / max(e0.elapsed_time(e1) / args.steps, 1e-3))], device=dev)
         if world > 1:   # data-parallel steps are collective: every rank must run the same number of them
