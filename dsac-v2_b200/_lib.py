@@ -132,6 +132,10 @@ SYMBOLS = {
     "dsact_cnn_replay_sample": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.POINTER(Batch), C.c_void_p]),
     "dsact_cnn_seed": (C.c_int, [C.c_void_p, C.c_uint64]),
     "dsact_cnn_step": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_int64, C.c_void_p]),
+    "dsact_cnn_grad_phase1": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_void_p]),
+    "dsact_cnn_grad_phase2": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
+    "dsact_cnn_compute_grads": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_void_p]),
+    "dsact_cnn_apply": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "dsact_cnn_read_stats": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "dsact_profile_step": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_int64, C.c_void_p, C.POINTER(Profile)]),
     "dsact_launch_count": (C.c_int64, [C.c_void_p]),

@@ -12,6 +12,9 @@
 //   conv forwards: pi(s), pi'(s'), Q1/Q2 features of s (shared by the (s,a) and (s,a~) passes), Q1'/Q2' features of s'
 //   heads: pi, pi' -> sample -> Q_k(s,a), Q'_k(s',a'), mean head of Q_k(s,a~) -> loss -> head backward (critics: both
 //   heads; actor path: mean head, input gradient only) -> policy_grad -> policy heads backward -> conv backward x3 -> Adam.
+// The sequence is enqueued in three parts (phase 1 = every forward, phase 2 = losses + backward, apply = Adam + Polyak)
+// that dsact_cnn_step runs back to back and the split entry points (dsact_cnn_grad_phase1/2, _compute_grads, _apply) run
+// one at a time, for the gradient-message seam and data-parallel callers.
 #pragma once
 #include "conv.cuh"
 
@@ -83,6 +86,10 @@ struct dsact_cnn_handle {
   bool bound = false;
   uint64_t seed = 0x5DEECE66Dull;
   int64_t dev_iter = -1, launches = 0;
+  // minibatch and noise of the last dsact_cnn_grad_phase1, read by the dsact_cnn_grad_phase2 that follows it
+  dsact_batch pending{};
+  int pending_batch = 0;   // 0: no phase 1 awaits its phase 2
+  const float *pending_eps1 = nullptr, *pending_z3 = nullptr, *pending_z4 = nullptr;
   // arena (floats from the workspace base)
   int64_t convP[DSACT_MAX_CONV + 1], convT[DSACT_MAX_CONV + 1], convQ[4][DSACT_MAX_CONV + 1];   // activations 1..nconv
   CnnHeadBuf hb[14];   // 0,1 pi mean/ls; 2,3 pi'; 4..7 Q1,Q2 (s,a) mean/ls; 8..11 Q1',Q2'; 12,13 mean head of Q1,Q2 on (s,a~)
@@ -364,6 +371,262 @@ static void cnn_conv_backward(dsact_cnn_handle* h, const CnnGeom& g, const float
   c.check();
 }
 
+// ---- one DSAC-T step in three parts: forwards (phase 1) | losses + backward (phase 2) | Adam + Polyak (apply) ---------
+// dsact_cnn_step enqueues all three; the split entry points enqueue one each, so that a data-parallel caller can
+// all-reduce the critics' std sums after phase 1 and the gradients + logged sums after phase 2.
+struct CnnSpans {   // per-network slices of the flat buffers
+  float *Pq[2], *Ppi, *Tq[2], *Tpi, *Gq[2], *Gpi;
+  long long n_all;   // 2 * n_q + n_pi + 1
+};
+static CnnSpans cnn_spans(const dsact_cnn_handle* h) {
+  const int64_t nq = h->q.n;
+  float *P = h->buf.params, *T = h->buf.targets, *G = h->buf.grads;
+  return CnnSpans{{P, P + nq}, P + 2 * nq, {T, T + nq}, T + 2 * nq, {G, G + nq}, G + 2 * nq, 2 * nq + h->pi.n + 1};
+}
+// the encoders' outputs; without a conv stack (the MLP approximators with separate heads) the feature is the observation
+struct CnnFeatures { const float *P, *T, *Q[4]; bool enc; };
+static CnnFeatures cnn_features(const dsact_cnn_handle* h, const dsact_batch& bt) {
+  float* W = h->Wp();
+  const CnnGeom &q = h->q, &pi = h->pi;
+  const bool enc = pi.nconv > 0;
+  return CnnFeatures{enc ? W + h->convP[pi.nconv] : bt.obs, enc ? W + h->convT[pi.nconv] : bt.obs2,
+                     {enc ? W + h->convQ[0][q.nconv] : bt.obs, enc ? W + h->convQ[1][q.nconv] : bt.obs,
+                      enc ? W + h->convQ[2][q.nconv] : bt.obs2, enc ? W + h->convQ[3][q.nconv] : bt.obs2},
+                     enc};
+}
+static StepScalars cnn_scalars(const dsact_cnn_handle* h, int64_t global_batch) {
+  StepScalars sc;
+  sc.tau_b = (float)h->cfg.tau_b; sc.alpha_fixed = (float)h->cfg.alpha_fixed; sc.inv_global_batch = (float)(1.0 / (double)global_batch);
+  sc.auto_alpha = h->cfg.auto_alpha; sc.log_alpha = h->buf.params + 2 * h->q.n + h->pi.n;
+  return sc;
+}
+
+// clears grads / accumulators, draws the noise (noise == null), runs every forward; sample_kernel leaves the local
+// critic-std sums in state[ST_STDSUM..+1].  Records the minibatch and noise for phase 2.
+static void cnn_enqueue_phase1(dsact_cnn_handle* h, const dsact_batch& bt, const dsact_noise* noise, Ctx& c) {
+  const dsact_cnn_config& cf = h->cfg;
+  const CnnGeom &q = h->q, &pi = h->pi;
+  const int B = bt.batch, A = cf.act_dim;
+  float* W = h->Wp();
+  const CnnSpans sp = cnn_spans(h);
+  {
+    int blocks = (int)((sp.n_all / 4 + 255) / 256); if (blocks > 2 * h->num_sms) blocks = 2 * h->num_sms; if (blocks < 1) blocks = 1;
+    launch_k(begin_step_kernel, blocks, 256, 0, c, h->buf.state, h->buf.grads, sp.n_all); c.done();
+  }
+  const float *eps1, *eps2;
+  if (noise) { eps1 = noise->eps1; eps2 = noise->eps2; h->pending_z3 = noise->z3; h->pending_z4 = noise->z4; }
+  else {
+    const int total = (B * A + 1) / 2 * 2 + (B + 1) / 2 * 2;
+    int blocks = (total / 2 + 255) / 256; if (blocks < 1) blocks = 1;
+    launch_k(noise_kernel, blocks, 256, 0, c, W + h->eps1, W + h->eps2, W + h->z3, W + h->z4, B, A, h->seed, (const float*)h->buf.state); c.done();
+    eps1 = W + h->eps1; eps2 = W + h->eps2; h->pending_z3 = W + h->z3; h->pending_z4 = W + h->z4;
+  }
+  h->pending_eps1 = eps1;
+
+  // ---- encoders: pi(s), pi'(s'), Q_k features of s, Q'_k features of s'
+  cnn_conv_forward(h, pi, sp.Ppi, bt.obs, h->convP, B, c);
+  cnn_conv_forward(h, pi, sp.Tpi, bt.obs2, h->convT, B, c);
+  for (int k = 0; k < 2; ++k) {
+    cnn_conv_forward(h, q, sp.Pq[k], bt.obs, h->convQ[k], B, c);
+    cnn_conv_forward(h, q, sp.Tq[k], bt.obs2, h->convQ[2 + k], B, c);
+  }
+  const CnnFeatures f = cnn_features(h, bt);
+
+  // ---- policy heads: logits = (mean | log_std), the layout sample_kernel reads (networks/cnn.py:233-240)
+  {
+    std::vector<CnnHeadFwd> v;
+    for (int hd = 0; hd < pi.nheads; ++hd) {
+      v.push_back({sp.Ppi + pi.head_off[hd], f.P, pi.F, nullptr, 0, &h->hb[hd], true, W + h->logitsP + hd * A, 2 * A});
+      v.push_back({sp.Tpi + pi.head_off[hd], f.T, pi.F, nullptr, 0, &h->hb[2 + hd], false, W + h->logitsT + hd * A, 2 * A});
+    }
+    cnn_heads_forward(h, pi.head, v, B, c);
+    if (pi.ls_row >= 0) {   // std_type "parameter": log_std columns = the learnable row
+      int blocks = (B * A + 255) / 256; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
+      launch_k(bcast_row_kernel, blocks, 256, 0, c, W + h->logitsP, 2 * A, A, (const float*)(sp.Ppi + pi.ls_row), B, A); c.done();
+      launch_k(bcast_row_kernel, blocks, 256, 0, c, W + h->logitsT, 2 * A, A, (const float*)(sp.Tpi + pi.ls_row), B, A); c.done();
+    }
+  }
+  // ---- critics on (s, a): out = (mean, raw std) packed [B,2] (networks/cnn.py:454-461; softplus is applied by the loss kernels)
+  {
+    std::vector<CnnHeadFwd> v;
+    for (int k = 0; k < 2; ++k)
+      for (int hd = 0; hd < q.nheads; ++hd)
+        v.push_back({sp.Pq[k] + q.head_off[hd], f.Q[k], q.F, bt.act, A, &h->hb[4 + 2 * k + hd], true, W + h->outQ[k] + hd, 2});
+    cnn_heads_forward(h, q.head, v, B, c);
+  }
+  {
+    SampleArgs a;
+    a.logits[0] = W + h->logitsP; a.logits[1] = W + h->logitsT;
+    a.eps[0] = eps1; a.eps[1] = eps2;
+    a.act[0] = W + h->new_act; a.act[1] = W + h->act2;
+    a.logp[0] = W + h->logp_new; a.logp[1] = W + h->logp2;
+    a.hi = h->buf.act_high; a.lo = h->buf.act_low; a.state = h->buf.state;
+    a.B = B; a.A = A; a.min_log_std = (float)cf.min_log_std; a.max_log_std = (float)cf.max_log_std; a.gauss = cf.act_dist;
+    a.img[0] = ImgOut{nullptr, 0, 1, 0}; a.img[1] = ImgOut{nullptr, 0, 1, 0};
+    a.out_q[0] = W + h->outQ[0]; a.out_q[1] = W + h->outQ[1];
+    a.advance_rng = noise ? 0 : 1;
+    int blocks = (B + 7) / 8; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
+    launch_k(sample_kernel, dim3(blocks, 2), 256, 0, c, a); c.done();
+  }
+  // ---- targets on (s', a') and the mean heads of the critics on (s, a~)
+  {
+    std::vector<CnnHeadFwd> v;
+    for (int k = 0; k < 2; ++k)
+      for (int hd = 0; hd < q.nheads; ++hd)
+        v.push_back({sp.Tq[k] + q.head_off[hd], f.Q[2 + k], q.F, W + h->act2, A, &h->hb[8 + 2 * k + hd], false, W + h->outQ[2 + k] + hd, 2});
+    for (int k = 0; k < 2; ++k)
+      v.push_back({sp.Pq[k] + q.head_off[0], f.Q[k], q.F, W + h->new_act, A, &h->hb[12 + k], true, W + h->outQ[4 + k], 2});
+    cnn_heads_forward(h, q.head, v, B, c);
+  }
+  h->pending = bt;
+  h->pending_batch = B;
+}
+
+// losses over `global_batch` rows (the local shard is h->pending), every backward pass, and the phase-2 tail: the
+// log_alpha gradient of the shard, the commit of the mean_std EMA and the temperature, the Adam scalars of the step
+static int cnn_enqueue_phase2(dsact_cnn_handle* h, int64_t global_batch, Ctx& c) {
+  const dsact_cnn_config& cf = h->cfg;
+  const CnnGeom &q = h->q, &pi = h->pi;
+  const dsact_batch& bt = h->pending;
+  const int B = bt.batch, A = cf.act_dim;
+  float* W = h->Wp();
+  const CnnSpans sp = cnn_spans(h);
+  const CnnFeatures f = cnn_features(h, bt);
+  const float* eps1 = h->pending_eps1;
+
+  // ---- losses and head-output gradients
+  const StepScalars sc = cnn_scalars(h, global_batch);
+  {
+    LossArgs a;
+    a.sc = sc;
+    a.rew = bt.rew; a.done = bt.done; a.z3 = h->pending_z3; a.z4 = h->pending_z4;
+    a.logp2 = W + h->logp2; a.logp_new = W + h->logp_new;
+    for (int k = 0; k < 2; ++k) {
+      a.out_q[k] = W + h->outQ[k]; a.out_qt[k] = W + h->outQ[2 + k]; a.out_qa[k] = W + h->outQ[4 + k];
+      a.d_out_q[k] = W + h->dOut[k]; a.d_out_qa[k] = W + h->dOut[4 + k];
+      a.gbias_q[k] = sp.Gq[k] + q.head_off[0] + q.head.b[q.head.L];          // output bias of the mean head
+      a.gbias_q_raw[k] = q.nheads == 2 ? sp.Gq[k] + q.head_off[1] + q.head.b[q.head.L] : nullptr;   // ... of the std head (one head: the next element)
+      a.img_q[k] = ImgOut{nullptr, 0, 1, 0}; a.img_qa[k] = ImgOut{nullptr, 0, 1, 0};
+    }
+    a.state = h->buf.state; a.B = B; a.gamma = (float)cf.gamma; a.inv_global_batch = sc.inv_global_batch;
+    int blocks = (B + 63) / 64; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
+    launch_k(loss_kernel, blocks, 64, 0, c, a); c.done();
+  }
+  auto zero = [&](float* p, long long n) {
+    int blocks = (int)((n + 255) / 256); if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms; if (blocks < 1) blocks = 1;
+    launch_k(zero_kernel, blocks, 256, 0, c, p, n); c.done();
+  };
+  zero(W + h->dfeat[0], (long long)B * pi.F);
+  zero(W + h->dfeat[1], (long long)B * q.F);
+  zero(W + h->dfeat[2], (long long)B * q.F);
+  zero(W + h->dfa[0], (long long)B * (q.F + A));
+  zero(W + h->dfa[1], (long long)B * (q.F + A));
+  // ---- critic backward through both heads (feature gradient accumulated over the heads), actor path through the mean head
+  {
+    std::vector<CnnHeadBwd> v;
+    for (int k = 0; k < 2; ++k)
+      for (int hd = 0; hd < q.nheads; ++hd)   // d(feature|act): only the feature part is used (replayed actions carry no gradient)
+        v.push_back({sp.Pq[k] + q.head_off[hd], sp.Gq[k] + q.head_off[hd], f.Q[k], q.F, bt.act, A, &h->hb[4 + 2 * k + hd],
+                     W + h->dOut[k] + hd, 2, nullptr});
+    for (int k = 0; k < 2; ++k)
+      v.push_back({sp.Pq[k] + q.head_off[0], nullptr, f.Q[k], q.F, W + h->new_act, A, &h->hb[12 + k], W + h->dOut[4 + k], 2, W + h->dfa[k]});
+    cnn_heads_backward(h, q.head, v, B, c);
+  }
+  // feature gradients of the critics: the layer-0 input gradient of both heads, feature columns only.  The generic
+  // backward above skipped it for the critic passes (din = null): do it here with the feature-width problem
+  for (int k = 0; k < 2 && f.enc; ++k) {
+    GemmGroup gd;
+    gd.n = 0;
+    for (int hd = 0; hd < q.nheads; ++hd) {
+      GemmProb p = prob_zero();
+      const Net& net = q.head;
+      p.A[0] = W + h->hb[4 + 2 * k + hd].dz[0]; p.lda[0] = net.s[1]; p.K[0] = net.s[1];
+      p.B[0] = sp.Pq[k] + q.head_off[hd] + net.w[0]; p.ldb[0] = net.s[0];
+      p.M = B; p.N = q.F; p.C = W + h->dfeat[1 + k]; p.ldc = q.F; p.epi = EPI_ATOMIC;
+      gd.p[gd.n++] = p;
+    }
+    launch_simt(h->num_sms, gd, V_DGRAD, c); c.done();
+  }
+  // dL/da~ through critic k = the action columns of dfa[k]: compact them for policy_grad_kernel
+  for (int k = 0; k < 2; ++k) {
+    CUDA_TRY(cudaMemcpy2DAsync(W + h->dAct[k], sizeof(float) * A, W + h->dfa[k] + q.F, sizeof(float) * (q.F + A), sizeof(float) * A, B,
+                               cudaMemcpyDeviceToDevice, c.s));
+  }
+  {
+    PolicyGradArgs a;
+    a.logits = W + h->logitsP; a.eps = eps1; a.d_act1 = W + h->dAct[0]; a.d_act2 = W + h->dAct[1];
+    a.hi = h->buf.act_high; a.lo = h->buf.act_low;
+    a.d_logits = W + h->dlogits; a.state = h->buf.state;
+    a.gbias = sp.Gpi + pi.head_off[0] + pi.head.b[pi.head.L];        // output bias of the mean head [A]
+    a.gbias_ls = pi.ls_row >= 0 ? sp.Gpi + pi.ls_row : (pi.nheads == 2 ? sp.Gpi + pi.head_off[1] + pi.head.b[pi.head.L] : nullptr);   // log_std head / row [A]
+    a.B = B; a.A = A; a.min_log_std = (float)cf.min_log_std; a.max_log_std = (float)cf.max_log_std; a.gauss = cf.act_dist;
+    a.inv_global_batch = sc.inv_global_batch;
+    a.img = ImgOut{nullptr, 0, 1, 0};
+    a.sc = sc;
+    int blocks = (B + 7) / 8; if (blocks > 8 * h->num_sms) blocks = 8 * h->num_sms; if (blocks < 1) blocks = 1;
+    launch_k(policy_grad_kernel, blocks, 256, sizeof(float) * 2 * A, c, a); c.done();
+  }
+  {
+    std::vector<CnnHeadBwd> v;
+    for (int hd = 0; hd < pi.nheads; ++hd)
+      v.push_back({sp.Ppi + pi.head_off[hd], sp.Gpi + pi.head_off[hd], f.P, pi.F, nullptr, 0, &h->hb[hd], W + h->dlogits + hd * A, 2 * A,
+                   f.enc ? W + h->dfeat[0] : nullptr});
+    cnn_heads_backward(h, pi.head, v, B, c);
+  }
+  // ---- encoders backward
+  if (f.enc) {
+    cnn_conv_backward(h, pi, sp.Ppi, sp.Gpi, bt.obs, h->convP, W + h->dfeat[0], B, c);
+    for (int k = 0; k < 2; ++k) cnn_conv_backward(h, q, sp.Pq[k], sp.Gq[k], bt.obs, h->convQ[k], W + h->dfeat[1 + k], B, c);
+  }
+
+  // ---- end of backward bookkeeping (log_alpha gradient over the local rows, EMA / temperature commit, Adam scalars)
+  const AdamHyper hy{cf.lr_q, cf.lr_pi, cf.lr_alpha, cf.adam_beta1, cf.adam_beta2};
+  launch_k(phase2_tail_kernel, 1, 32, 0, c, sp.Gpi + pi.n, h->buf.state, sc, -(float)cf.act_dim, B, hy, 1); c.done();
+  h->pending_batch = 0;
+  return DSACT_OK;
+}
+
+// Adam on the three spans + log_alpha, delayed Polyak, step counters.  `scalars_ready` = 1: the phase-2 tail enqueued
+// just before (same counters) wrote the step's Adam scalars; 0: form them here (after a separate compute_grads, or when
+// `grads` was written from outside).
+static void cnn_enqueue_apply(dsact_cnn_handle* h, int scalars_ready, Ctx& c) {
+  const dsact_cnn_config& cf = h->cfg;
+  const CnnSpans sp = cnn_spans(h);
+  ApplyArgs a;
+  memset(&a, 0, sizeof(a));
+  a.params = h->buf.params; a.targets = h->buf.targets; a.grads = h->buf.grads; a.m = h->buf.adam_m; a.v = h->buf.adam_v;
+  a.state = h->buf.state;
+  a.n_q2 = 2 * h->q.n; a.n_all = sp.n_all;
+  a.delay_update = cf.delay_update; a.auto_alpha = cf.auto_alpha;
+  a.hy = AdamHyper{cf.lr_q, cf.lr_pi, cf.lr_alpha, cf.adam_beta1, cf.adam_beta2}; a.scalars_ready = scalars_ready;
+  a.eps = (float)cf.adam_eps; a.tau = (float)cf.tau;
+  a.omb1 = (float)(1.0 - cf.adam_beta1); a.b2f = (float)cf.adam_beta2; a.omb2 = (float)(1.0 - cf.adam_beta2);
+  a.g_lo = 0; a.g_hi = (sp.n_all + 3) / 4; a.finish = 1;
+  int blocks = (int)(((sp.n_all + 3) / 4 + 255) / 256); if (blocks > 8 * h->num_sms) blocks = 8 * h->num_sms;
+  launch_k(apply_kernel<0>, blocks, 256, 0, c, a); c.done();
+}
+
+static int cnn_check_batch(const dsact_cnn_handle* h, const dsact_batch* batch) {
+  if (!h || !h->bound) return fail(DSACT_ESTATE, "dsact_cnn_bind has not been called");
+  if (!batch || !batch->obs || !batch->act || !batch->rew || !batch->obs2 || !batch->done) return fail(DSACT_EINVAL, "null batch pointer");
+  if (batch->batch < 1 || batch->batch > h->cfg.max_batch) return fail(DSACT_EINVAL, "batch %d outside [1, max_batch=%d]", batch->batch, h->cfg.max_batch);
+  return DSACT_OK;
+}
+static int cnn_split_supported(const dsact_cnn_handle* h, const char* fn) {
+  if (h && h->cfg.algo == 1) return fail(DSACT_EINVAL, "%s: DSAC_V1 handles (algo = 1) have dsact_cnn_step only", fn);
+  return DSACT_OK;
+}
+static int cnn_sync_iteration(dsact_cnn_handle* h, int64_t iteration, cudaStream_t s) {
+  if (iteration < 0 || iteration > 0x7fffffff) return fail(DSACT_EINVAL, "iteration out of range");
+  if (h->dev_iter != iteration) { set_iter_kernel<<<1, 32, 0, s>>>(h->buf.state, (int)iteration); CUDA_TRY(cudaGetLastError()); }
+  return DSACT_OK;
+}
+static int cnn_finish(dsact_cnn_handle* h, const Ctx& c) {
+  if (c.err != cudaSuccess) return fail(DSACT_ECUDA, "kernel launch failed: %s", cudaGetErrorString(c.err));
+  h->launches += c.launches;
+  return DSACT_OK;
+}
+
 #include "v1_step.cuh"
 
 extern "C" {
@@ -414,6 +677,7 @@ int dsact_cnn_bind(dsact_cnn_handle* h, const dsact_buffers* b) {
   h->buf = *b;
   h->bound = true;
   h->dev_iter = -1;
+  h->pending_batch = 0;
   return DSACT_OK;
 }
 
@@ -500,207 +764,73 @@ int dsact_cnn_replay_sample(dsact_cnn_handle* h, int32_t batch, int64_t size, co
 }
 
 int dsact_cnn_step(dsact_cnn_handle* h, const dsact_batch* batch, const dsact_noise* noise, int64_t iteration, void* stream) {
-  if (!h || !h->bound) return fail(DSACT_ESTATE, "dsact_cnn_bind has not been called");
-  if (!batch || !batch->obs || !batch->act || !batch->rew || !batch->obs2 || !batch->done) return fail(DSACT_EINVAL, "null batch pointer");
-  if (batch->batch < 1 || batch->batch > h->cfg.max_batch) return fail(DSACT_EINVAL, "batch %d outside [1, max_batch=%d]", batch->batch, h->cfg.max_batch);
-  int rc = check_noise(noise);
-  if (rc) return rc;
+  int rc = cnn_check_batch(h, batch);
+  if (rc || (rc = check_noise(noise))) return rc;
   if (iteration < 0 || iteration > 0x7fffffff) return fail(DSACT_EINVAL, "iteration out of range");
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  if (h->dev_iter != iteration) { set_iter_kernel<<<1, 32, 0, s>>>(h->buf.state, (int)iteration); CUDA_TRY(cudaGetLastError()); }
-  const dsact_cnn_config& cf = h->cfg;
-  if (cf.algo == 1) return cnn_step_v1(h, batch, noise, iteration, s);
-  const CnnGeom &q = h->q, &pi = h->pi;
-  const int B = batch->batch, A = cf.act_dim;
-  float* W = h->Wp();
-  float* P = h->buf.params; float* T = h->buf.targets; float* G = h->buf.grads;
-  float* Pq[2] = {P, P + q.n}; float* Ppi = P + 2 * q.n;
-  float* Tq[2] = {T, T + q.n}; float* Tpi = T + 2 * q.n;
-  float* Gq[2] = {G, G + q.n}; float* Gpi = G + 2 * q.n;
+  if ((rc = cnn_sync_iteration(h, iteration, s))) return rc;
+  if (h->cfg.algo == 1) return cnn_step_v1(h, batch, noise, iteration, s);
   Ctx c{s, 0, cudaSuccess};
   c.pdl = false;
-  const long long n_all = 2 * q.n + pi.n + 1;
-  {
-    int blocks = (int)((n_all / 4 + 255) / 256); if (blocks > 2 * h->num_sms) blocks = 2 * h->num_sms; if (blocks < 1) blocks = 1;
-    launch_k(begin_step_kernel, blocks, 256, 0, c, h->buf.state, G, n_all); c.done();
-  }
-  const float *eps1, *eps2, *z3, *z4;
-  if (noise) { eps1 = noise->eps1; eps2 = noise->eps2; z3 = noise->z3; z4 = noise->z4; }
-  else {
-    const int total = (B * A + 1) / 2 * 2 + (B + 1) / 2 * 2;
-    int blocks = (total / 2 + 255) / 256; if (blocks < 1) blocks = 1;
-    launch_k(noise_kernel, blocks, 256, 0, c, W + h->eps1, W + h->eps2, W + h->z3, W + h->z4, B, A, h->seed, (const float*)h->buf.state); c.done();
-    eps1 = W + h->eps1; eps2 = W + h->eps2; z3 = W + h->z3; z4 = W + h->z4;
-  }
+  cnn_enqueue_phase1(h, *batch, noise, c);
+  rc = cnn_enqueue_phase2(h, batch->batch, c);
+  if (rc) { h->pending_batch = 0; return rc; }
+  cnn_enqueue_apply(h, 1, c);
+  if ((rc = cnn_finish(h, c))) return rc;
+  h->dev_iter = iteration + 1;
+  return DSACT_OK;
+}
 
-  // ---- encoders: pi(s), pi'(s'), Q_k features of s, Q'_k features of s'
-  cnn_conv_forward(h, pi, Ppi, batch->obs, h->convP, B, c);
-  cnn_conv_forward(h, pi, Tpi, batch->obs2, h->convT, B, c);
-  for (int k = 0; k < 2; ++k) {
-    cnn_conv_forward(h, q, Pq[k], batch->obs, h->convQ[k], B, c);
-    cnn_conv_forward(h, q, Tq[k], batch->obs2, h->convQ[2 + k], B, c);
-  }
-  // without a conv stack (the MLP approximators with separate heads) the feature is the observation itself
-  const bool enc = pi.nconv > 0;
-  const float* featP = enc ? W + h->convP[pi.nconv] : batch->obs;
-  const float* featT = enc ? W + h->convT[pi.nconv] : batch->obs2;
-  const float* featQ[4] = {enc ? W + h->convQ[0][q.nconv] : batch->obs, enc ? W + h->convQ[1][q.nconv] : batch->obs,
-                           enc ? W + h->convQ[2][q.nconv] : batch->obs2, enc ? W + h->convQ[3][q.nconv] : batch->obs2};
+int dsact_cnn_grad_phase1(dsact_cnn_handle* h, const dsact_batch* batch, const dsact_noise* noise, void* stream) {
+  int rc = cnn_check_batch(h, batch);
+  if (rc || (rc = check_noise(noise)) || (rc = cnn_split_supported(h, "dsact_cnn_grad_phase1"))) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  Ctx c{(cudaStream_t)stream, 0, cudaSuccess};
+  c.pdl = false;
+  cnn_enqueue_phase1(h, *batch, noise, c);
+  if ((rc = cnn_finish(h, c))) h->pending_batch = 0;
+  return rc;
+}
 
-  // ---- policy heads: logits = (mean | log_std), the layout sample_kernel reads (networks/cnn.py:233-240)
-  {
-    std::vector<CnnHeadFwd> v;
-    for (int hd = 0; hd < pi.nheads; ++hd) {
-      v.push_back({Ppi + pi.head_off[hd], featP, pi.F, nullptr, 0, &h->hb[hd], true, W + h->logitsP + hd * A, 2 * A});
-      v.push_back({Tpi + pi.head_off[hd], featT, pi.F, nullptr, 0, &h->hb[2 + hd], false, W + h->logitsT + hd * A, 2 * A});
-    }
-    cnn_heads_forward(h, pi.head, v, B, c);
-    if (pi.ls_row >= 0) {   // std_type "parameter": log_std columns = the learnable row
-      int blocks = (B * A + 255) / 256; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
-      launch_k(bcast_row_kernel, blocks, 256, 0, c, W + h->logitsP, 2 * A, A, (const float*)(Ppi + pi.ls_row), B, A); c.done();
-      launch_k(bcast_row_kernel, blocks, 256, 0, c, W + h->logitsT, 2 * A, A, (const float*)(Tpi + pi.ls_row), B, A); c.done();
-    }
-  }
-  // ---- critics on (s, a): out = (mean, raw std) packed [B,2] (networks/cnn.py:454-461; softplus is applied by the loss kernels)
-  {
-    std::vector<CnnHeadFwd> v;
-    for (int k = 0; k < 2; ++k)
-      for (int hd = 0; hd < q.nheads; ++hd)
-        v.push_back({Pq[k] + q.head_off[hd], featQ[k], q.F, batch->act, A, &h->hb[4 + 2 * k + hd], true, W + h->outQ[k] + hd, 2});
-    cnn_heads_forward(h, q.head, v, B, c);
-  }
-  {
-    SampleArgs a;
-    a.logits[0] = W + h->logitsP; a.logits[1] = W + h->logitsT;
-    a.eps[0] = eps1; a.eps[1] = eps2;
-    a.act[0] = W + h->new_act; a.act[1] = W + h->act2;
-    a.logp[0] = W + h->logp_new; a.logp[1] = W + h->logp2;
-    a.hi = h->buf.act_high; a.lo = h->buf.act_low; a.state = h->buf.state;
-    a.B = B; a.A = A; a.min_log_std = (float)cf.min_log_std; a.max_log_std = (float)cf.max_log_std; a.gauss = cf.act_dist;
-    a.img[0] = ImgOut{nullptr, 0, 1, 0}; a.img[1] = ImgOut{nullptr, 0, 1, 0};
-    a.out_q[0] = W + h->outQ[0]; a.out_q[1] = W + h->outQ[1];
-    a.advance_rng = noise ? 0 : 1;
-    int blocks = (B + 7) / 8; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
-    launch_k(sample_kernel, dim3(blocks, 2), 256, 0, c, a); c.done();
-  }
-  // ---- targets on (s', a') and the mean heads of the critics on (s, a~)
-  {
-    std::vector<CnnHeadFwd> v;
-    for (int k = 0; k < 2; ++k)
-      for (int hd = 0; hd < q.nheads; ++hd)
-        v.push_back({Tq[k] + q.head_off[hd], featQ[2 + k], q.F, W + h->act2, A, &h->hb[8 + 2 * k + hd], false, W + h->outQ[2 + k] + hd, 2});
-    for (int k = 0; k < 2; ++k)
-      v.push_back({Pq[k] + q.head_off[0], featQ[k], q.F, W + h->new_act, A, &h->hb[12 + k], true, W + h->outQ[4 + k], 2});
-    cnn_heads_forward(h, q.head, v, B, c);
-  }
+int dsact_cnn_grad_phase2(dsact_cnn_handle* h, int64_t global_batch, void* stream) {
+  if (!h || !h->bound) return fail(DSACT_ESTATE, "dsact_cnn_bind has not been called");
+  int rc = cnn_split_supported(h, "dsact_cnn_grad_phase2");
+  if (rc) return rc;
+  if (h->pending_batch < 1) return fail(DSACT_ESTATE, "dsact_cnn_grad_phase2 without a preceding dsact_cnn_grad_phase1");
+  if (global_batch < h->pending_batch || global_batch > 0x7fffffff)
+    return fail(DSACT_EINVAL, "global_batch %lld outside [local batch %d, 2^31)", (long long)global_batch, h->pending_batch);
+  CUDA_TRY(cudaSetDevice(h->device));
+  Ctx c{(cudaStream_t)stream, 0, cudaSuccess};
+  c.pdl = false;
+  rc = cnn_enqueue_phase2(h, global_batch, c);
+  h->pending_batch = 0;
+  return rc ? rc : cnn_finish(h, c);
+}
 
-  // ---- losses and head-output gradients
-  const float invB = (float)(1.0 / (double)B);
-  StepScalars sc;
-  sc.tau_b = (float)cf.tau_b; sc.alpha_fixed = (float)cf.alpha_fixed; sc.inv_global_batch = invB;
-  sc.auto_alpha = cf.auto_alpha; sc.log_alpha = P + 2 * q.n + pi.n;
-  {
-    LossArgs a;
-    a.sc = sc;
-    a.rew = batch->rew; a.done = batch->done; a.z3 = z3; a.z4 = z4;
-    a.logp2 = W + h->logp2; a.logp_new = W + h->logp_new;
-    for (int k = 0; k < 2; ++k) {
-      a.out_q[k] = W + h->outQ[k]; a.out_qt[k] = W + h->outQ[2 + k]; a.out_qa[k] = W + h->outQ[4 + k];
-      a.d_out_q[k] = W + h->dOut[k]; a.d_out_qa[k] = W + h->dOut[4 + k];
-      a.gbias_q[k] = Gq[k] + q.head_off[0] + q.head.b[q.head.L];          // output bias of the mean head
-      a.gbias_q_raw[k] = q.nheads == 2 ? Gq[k] + q.head_off[1] + q.head.b[q.head.L] : nullptr;   // ... of the std head (one head: the next element)
-      a.img_q[k] = ImgOut{nullptr, 0, 1, 0}; a.img_qa[k] = ImgOut{nullptr, 0, 1, 0};
-    }
-    a.state = h->buf.state; a.B = B; a.gamma = (float)cf.gamma; a.inv_global_batch = invB;
-    int blocks = (B + 63) / 64; if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms;
-    launch_k(loss_kernel, blocks, 64, 0, c, a); c.done();
-  }
-  auto zero = [&](float* p, long long n) {
-    int blocks = (int)((n + 255) / 256); if (blocks > 4 * h->num_sms) blocks = 4 * h->num_sms; if (blocks < 1) blocks = 1;
-    launch_k(zero_kernel, blocks, 256, 0, c, p, n); c.done();
-  };
-  zero(W + h->dfeat[0], (long long)B * pi.F);
-  zero(W + h->dfeat[1], (long long)B * q.F);
-  zero(W + h->dfeat[2], (long long)B * q.F);
-  zero(W + h->dfa[0], (long long)B * (q.F + A));
-  zero(W + h->dfa[1], (long long)B * (q.F + A));
-  // ---- critic backward through both heads (feature gradient accumulated over the heads), actor path through the mean head
-  {
-    std::vector<CnnHeadBwd> v;
-    for (int k = 0; k < 2; ++k)
-      for (int hd = 0; hd < q.nheads; ++hd)   // d(feature|act): only the feature part is used (replayed actions carry no gradient)
-        v.push_back({Pq[k] + q.head_off[hd], Gq[k] + q.head_off[hd], featQ[k], q.F, batch->act, A, &h->hb[4 + 2 * k + hd],
-                     W + h->dOut[k] + hd, 2, nullptr});
-    for (int k = 0; k < 2; ++k)
-      v.push_back({Pq[k] + q.head_off[0], nullptr, featQ[k], q.F, W + h->new_act, A, &h->hb[12 + k], W + h->dOut[4 + k], 2, W + h->dfa[k]});
-    cnn_heads_backward(h, q.head, v, B, c);
-  }
-  // feature gradients of the critics: the layer-0 input gradient of both heads, feature columns only.  The generic
-  // backward above skipped it for the critic passes (din = null): do it here with the feature-width problem
-  for (int k = 0; k < 2 && enc; ++k) {
-    GemmGroup gd;
-    gd.n = 0;
-    for (int hd = 0; hd < q.nheads; ++hd) {
-      GemmProb p = prob_zero();
-      const Net& net = q.head;
-      p.A[0] = W + h->hb[4 + 2 * k + hd].dz[0]; p.lda[0] = net.s[1]; p.K[0] = net.s[1];
-      p.B[0] = Pq[k] + q.head_off[hd] + net.w[0]; p.ldb[0] = net.s[0];
-      p.M = B; p.N = q.F; p.C = W + h->dfeat[1 + k]; p.ldc = q.F; p.epi = EPI_ATOMIC;
-      gd.p[gd.n++] = p;
-    }
-    launch_simt(h->num_sms, gd, V_DGRAD, c); c.done();
-  }
-  // dL/da~ through critic k = the action columns of dfa[k]: compact them for policy_grad_kernel
-  for (int k = 0; k < 2; ++k) {
-    CUDA_TRY(cudaMemcpy2DAsync(W + h->dAct[k], sizeof(float) * A, W + h->dfa[k] + q.F, sizeof(float) * (q.F + A), sizeof(float) * A, B,
-                               cudaMemcpyDeviceToDevice, s));
-  }
-  {
-    PolicyGradArgs a;
-    a.logits = W + h->logitsP; a.eps = eps1; a.d_act1 = W + h->dAct[0]; a.d_act2 = W + h->dAct[1];
-    a.hi = h->buf.act_high; a.lo = h->buf.act_low;
-    a.d_logits = W + h->dlogits; a.state = h->buf.state;
-    a.gbias = Gpi + pi.head_off[0] + pi.head.b[pi.head.L];        // output bias of the mean head [A]
-    a.gbias_ls = pi.ls_row >= 0 ? Gpi + pi.ls_row : (pi.nheads == 2 ? Gpi + pi.head_off[1] + pi.head.b[pi.head.L] : nullptr);   // log_std head / row [A]
-    a.B = B; a.A = A; a.min_log_std = (float)cf.min_log_std; a.max_log_std = (float)cf.max_log_std; a.gauss = cf.act_dist;
-    a.inv_global_batch = invB;
-    a.img = ImgOut{nullptr, 0, 1, 0};
-    a.sc = sc;
-    int blocks = (B + 7) / 8; if (blocks > 8 * h->num_sms) blocks = 8 * h->num_sms; if (blocks < 1) blocks = 1;
-    launch_k(policy_grad_kernel, blocks, 256, sizeof(float) * 2 * A, c, a); c.done();
-  }
-  {
-    std::vector<CnnHeadBwd> v;
-    for (int hd = 0; hd < pi.nheads; ++hd)
-      v.push_back({Ppi + pi.head_off[hd], Gpi + pi.head_off[hd], featP, pi.F, nullptr, 0, &h->hb[hd], W + h->dlogits + hd * A, 2 * A,
-                   enc ? W + h->dfeat[0] : nullptr});
-    cnn_heads_backward(h, pi.head, v, B, c);
-  }
-  // ---- encoders backward
-  if (enc) {
-    cnn_conv_backward(h, pi, Ppi, Gpi, batch->obs, h->convP, W + h->dfeat[0], B, c);
-    for (int k = 0; k < 2; ++k) cnn_conv_backward(h, q, Pq[k], Gq[k], batch->obs, h->convQ[k], W + h->dfeat[1 + k], B, c);
-  }
+int dsact_cnn_compute_grads(dsact_cnn_handle* h, const dsact_batch* batch, const dsact_noise* noise, void* stream) {
+  int rc = cnn_check_batch(h, batch);
+  if (rc || (rc = check_noise(noise)) || (rc = cnn_split_supported(h, "dsact_cnn_compute_grads"))) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  Ctx c{(cudaStream_t)stream, 0, cudaSuccess};
+  c.pdl = false;
+  cnn_enqueue_phase1(h, *batch, noise, c);
+  rc = cnn_enqueue_phase2(h, batch->batch, c);
+  h->pending_batch = 0;
+  return rc ? rc : cnn_finish(h, c);
+}
 
-  // ---- end of backward bookkeeping + Adam / Polyak
-  AdamHyper hy{cf.lr_q, cf.lr_pi, cf.lr_alpha, cf.adam_beta1, cf.adam_beta2};
-  launch_k(phase2_tail_kernel, 1, 32, 0, c, G + 2 * q.n + pi.n, h->buf.state, sc, -(float)cf.act_dim, B, hy, 1); c.done();
-  {
-    ApplyArgs a;
-    memset(&a, 0, sizeof(a));
-    a.params = P; a.targets = T; a.grads = G; a.m = h->buf.adam_m; a.v = h->buf.adam_v; a.state = h->buf.state;
-    a.n_q2 = 2 * q.n; a.n_all = n_all;
-    a.delay_update = cf.delay_update; a.auto_alpha = cf.auto_alpha;
-    a.hy = hy; a.scalars_ready = 1;
-    a.eps = (float)cf.adam_eps; a.tau = (float)cf.tau;
-    a.omb1 = (float)(1.0 - cf.adam_beta1); a.b2f = (float)cf.adam_beta2; a.omb2 = (float)(1.0 - cf.adam_beta2);
-    a.g_lo = 0; a.g_hi = (n_all + 3) / 4; a.finish = 1;
-    int blocks = (int)(((n_all + 3) / 4 + 255) / 256); if (blocks > 8 * h->num_sms) blocks = 8 * h->num_sms;
-    launch_k(apply_kernel<0>, blocks, 256, 0, c, a); c.done();
-  }
-  if (c.err != cudaSuccess) return fail(DSACT_ECUDA, "kernel launch failed: %s", cudaGetErrorString(c.err));
-  h->launches += c.launches;
+int dsact_cnn_apply(dsact_cnn_handle* h, int64_t iteration, void* stream) {
+  if (!h || !h->bound) return fail(DSACT_ESTATE, "dsact_cnn_bind has not been called");
+  int rc = cnn_split_supported(h, "dsact_cnn_apply");
+  if (rc) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = cnn_sync_iteration(h, iteration, s))) return rc;
+  Ctx c{s, 0, cudaSuccess};
+  c.pdl = false;
+  cnn_enqueue_apply(h, 0, c);
+  if ((rc = cnn_finish(h, c))) return rc;
   h->dev_iter = iteration + 1;
   return DSACT_OK;
 }

@@ -11,7 +11,8 @@ Two transports.  `connect_peers` + `engine.dp_step`: the exchanges run inside th
 kernels over NVLink peer memory (CUDA IPC), the whole data-parallel step is one graph launch
 per rank.  `data_parallel_gradients`: the same seam through `torch.distributed` (NCCL on
 GPUs; gloo in the CPU tests) — the fallback, and the path of the split gradient API.  `engine` is anything with grad_phase1 / grad_phase2 / state / grads — the CUDA
-`Engine`, or a CPU stand-in in tests/test_dp_gloo.py.
+`Engine`, the head-wise `CnnEngine` (which has no peer-memory exchange: this is its only data-parallel path), or a
+CPU stand-in in tests/test_dp_gloo.py.
 """
 from __future__ import annotations
 

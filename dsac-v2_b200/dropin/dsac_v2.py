@@ -11,6 +11,10 @@ the B200 engine (libdsact.so) instead of eager PyTorch.
 * `get_remote_update_info` / `remote_update` keep the gradient-message seam
   (reference :107-138); with `torch.distributed` initialised the step is
   data-parallel (all-reduce of the two critic-std sums and of the flat gradients).
+  Both hold for every configuration: the MLP approximators on the tcgen05 engine,
+  and the CNN approximators / policy std types mlp_separated and parameter on the
+  head-wise engine (whose data-parallel exchange is torch.distributed only, so
+  `dsact_dp_transport="peer"` means NCCL for those configurations).
 
 Extra kwargs (all optional): `dsact_noise` = "device" (Philox on the GPU, default)
 or "reference" (draw the 8 normals of one update from torch's CPU generator in the
@@ -262,7 +266,9 @@ class DSAC_V2:
             raise ValueError("dsact_noise must be 'device' or 'reference'")
         self.data_parallel = kwargs.get("dsact_data_parallel", True)
         # "peer": exchanges inside the step's kernels over NVLink peer memory (falls back to NCCL if the ranks cannot
-        # map each other's buffers); "nccl": torch.distributed all-reduces between three graph launches
+        # map each other's buffers); "nccl": torch.distributed all-reduces between three graph launches.  The head-wise
+        # engine (CNN approximators, policy std types mlp_separated / parameter) has no peer-memory exchange: for those
+        # configurations both values mean torch.distributed all-reduces between its phase launches
         self.dp_transport = kwargs.get("dsact_dp_transport", "peer")
         self._peer_dp, self._peer_eng = None, None
         self._slots, self._owners, self._cursor = None, [None] * self._RING, 0
@@ -358,12 +364,13 @@ class DSAC_V2:
         if world == 1:
             eng.step(data, iteration, self._noise(B))
             return self._stats(eng, B, t0)
-        if self._peer_dp is None or self._peer_eng is not eng:   # first data-parallel update (or the engine was rebuilt):
-            self._peer_dp = self.dp_transport != "nccl" and dp.connect_peers(eng, dist)   # map the exchange buffers (collective)
-            self._peer_eng = eng
-        if self._peer_dp:           # one graph launch; exchanges inside the step's kernels over NVLink peer memory
-            eng.dp_step(data, iteration, B * world, self._noise(B))
-            return self._stats(eng, B * world, t0)
+        if not self.networks._cnn:   # the tcgen05 engine; the head-wise engine exchanges through torch.distributed only
+            if self._peer_dp is None or self._peer_eng is not eng:   # first data-parallel update (or the engine was rebuilt):
+                self._peer_dp = self.dp_transport != "nccl" and dp.connect_peers(eng, dist)   # map the exchange buffers (collective)
+                self._peer_eng = eng
+            if self._peer_dp:           # one graph launch; exchanges inside the step's kernels over NVLink peer memory
+                eng.dp_step(data, iteration, B * world, self._noise(B))
+                return self._stats(eng, B * world, t0)
         gb = self._gradients(data, eng)
         eng.apply(iteration)
         return self._stats(eng, gb, t0)

@@ -165,23 +165,55 @@ class CnnEngine:
         return out
 
     # ---- the path -------------------------------------------------------------------------------------------------------
+    def _batch(self, data: Dict[str, torch.Tensor]) -> Batch:
+        """Device copies of the minibatch (kept alive on the engine until the next call that reads them) as a Batch."""
+        t = {k: data[k].to(device=self.device, dtype=torch.float32).contiguous() for k in ("obs", "act", "rew", "obs2", "done")}
+        B = t["obs"].shape[0]
+        c = self.cfg
+        if t["obs"][0].numel() != self.obs_elems or t["obs2"].shape != t["obs"].shape or t["act"].shape != (B, c.act_dim):
+            raise ValueError("minibatch shapes do not match the configured observation / action shape")
+        self._keep = t
+        return Batch(t["obs"].data_ptr(), t["act"].data_ptr(), t["rew"].data_ptr(), t["obs2"].data_ptr(), t["done"].data_ptr(), B, None)
+
+    def _noise(self, noise):
+        """eps1, eps2, z3, z4 on the device as a Noise pointer, or None (the engine draws them)."""
+        if noise is None:
+            return None
+        nz = [torch.as_tensor(x).to(device=self.device, dtype=torch.float32).contiguous() for x in noise]
+        self._keep_noise = nz
+        return C.byref(Noise(*(x.data_ptr() for x in nz)))
+
     def step(self, data: Dict[str, torch.Tensor], iteration: int, noise=None):
         """DSAC_V2.local_update (reference dsac_v2.py:102-105) with image observations [B, C, H, W] on the device."""
         with torch.cuda.device(self.device):
-            t = {k: data[k].to(device=self.device, dtype=torch.float32).contiguous() for k in ("obs", "act", "rew", "obs2", "done")}
-            B = t["obs"].shape[0]
-            c = self.cfg
-            if t["obs"][0].numel() != self.obs_elems or t["obs2"].shape != t["obs"].shape or t["act"].shape != (B, c.act_dim):
-                raise ValueError("minibatch shapes do not match the configured observation / action shape")
-            b = Batch(t["obs"].data_ptr(), t["act"].data_ptr(), t["rew"].data_ptr(), t["obs2"].data_ptr(), t["done"].data_ptr(), B, None)
-            n = None
-            if noise is not None:
-                nz = [torch.as_tensor(x).to(device=self.device, dtype=torch.float32).contiguous() for x in noise]
-                n = C.byref(Noise(*(x.data_ptr() for x in nz)))
-                self._keep_noise = nz
-            self._keep = t
-            check(self.lib.dsact_cnn_step(self.h, C.byref(b), n, int(iteration), self._stream()))
-        self.last_batch = B
+            b = self._batch(data)
+            check(self.lib.dsact_cnn_step(self.h, C.byref(b), self._noise(noise), int(iteration), self._stream()))
+        self.last_batch = b.batch
+
+    # ---- split form: the gradient-message seam and data-parallel steps (dp.data_parallel_gradients) -------------------
+    def grad_phase1(self, data: Dict[str, torch.Tensor], noise=None):
+        """Every forward of the step on the local minibatch; leaves the local critic-std sums in state[4:6]."""
+        with torch.cuda.device(self.device):
+            b = self._batch(data)
+            check(self.lib.dsact_cnn_grad_phase1(self.h, C.byref(b), self._noise(noise), self._stream()))
+        self.last_batch = b.batch
+
+    def grad_phase2(self, global_batch: int):
+        """Losses (means over `global_batch` rows) and every backward pass of the minibatch of grad_phase1."""
+        with torch.cuda.device(self.device):
+            check(self.lib.dsact_cnn_grad_phase2(self.h, int(global_batch), self._stream()))
+
+    def compute_grads(self, data: Dict[str, torch.Tensor], noise=None):
+        """grad_phase1 + grad_phase2 over this minibatch alone: `grads` holds the step's gradients."""
+        with torch.cuda.device(self.device):
+            b = self._batch(data)
+            check(self.lib.dsact_cnn_compute_grads(self.h, C.byref(b), self._noise(noise), self._stream()))
+        self.last_batch = b.batch
+
+    def apply(self, iteration: int):
+        """Adam + delayed Polyak with whatever `grads` holds (DSAC_V2.remote_update)."""
+        with torch.cuda.device(self.device):
+            check(self.lib.dsact_cnn_apply(self.h, int(iteration), self._stream()))
 
     # ---- device replay ring (flattened image rows) ---------------------------------------------------------------------
     @property

@@ -258,6 +258,24 @@ int dsact_cnn_set_carry(dsact_cnn_handle *h, float mean_std1, float mean_std2, i
                         void *stream);
 int dsact_cnn_seed(dsact_cnn_handle *h, uint64_t seed);
 int dsact_cnn_step(dsact_cnn_handle *h, const dsact_batch *batch, const dsact_noise *noise, int64_t iteration, void *stream);
+/* Split form of dsact_cnn_step, with the contracts of dsact_grad_phase1 / _phase2 / dsact_compute_grads / dsact_apply
+ * (get_remote_update_info / remote_update, dsac_v2.py:107-138, and data-parallel updates through torch.distributed):
+ *  phase1: clears grads and accumulators, draws the noise on the device if `noise` is NULL, runs every forward; leaves
+ *          the LOCAL per-critic sums of std in state[DSACT_STATE_STDSUM..+1].  The handle keeps the batch / noise
+ *          pointers until the phase2 that follows, so they must stay valid until then;
+ *  phase2: mean_std EMA, losses with means over `global_batch` rows (>= the phase-1 batch, else DSACT_EINVAL), every
+ *          backward pass, the log_alpha gradient of the local rows, the EMA / temperature commit.  Without a preceding
+ *          phase1: DSACT_ESTATE.  A data-parallel caller all-reduces the two std sums between the phases, and `grads`
+ *          + the logged accumulators (16 sums, then 2 minima at DSACT_STATE_ACC + 16) after phase2;
+ *  compute_grads = phase1 + phase2 with global_batch = the batch;
+ *  apply: Adam on the three networks and log_alpha + delayed Polyak on whatever is in `grads` (it may have been
+ *         overwritten by the caller), for `iteration`.
+ * dsact_cnn_step = phase1 + phase2(batch) + apply, enqueued by the same code.  On a DSAC_V1 handle (algo = 1) the four
+ * return DSACT_EINVAL. */
+int dsact_cnn_grad_phase1(dsact_cnn_handle *h, const dsact_batch *batch, const dsact_noise *noise, void *stream);
+int dsact_cnn_grad_phase2(dsact_cnn_handle *h, int64_t global_batch, void *stream);
+int dsact_cnn_compute_grads(dsact_cnn_handle *h, const dsact_batch *batch, const dsact_noise *noise, void *stream);
+int dsact_cnn_apply(dsact_cnn_handle *h, int64_t iteration, void *stream);
 int dsact_cnn_read_stats(dsact_cnn_handle *h, int64_t global_batch, float *host_out, void *stream);
 /* device replay ring for image transitions: rows of obs / obs2 are the flattened [C*H*W] images (fp32, like the
  * reference's CarRacing data, env_gym/gym_carracing_data.py:19-21); same semantics as dsact_replay_bind / _add / _sample */
