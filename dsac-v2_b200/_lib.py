@@ -91,6 +91,12 @@ class Replay(C.Structure):
                 ("capacity", C.c_int64)]
 
 
+class ReplayU8(C.Structure):
+    """dsact_replay_u8: obs / obs2 hold one uint8 code per pixel (the pixel is float32(k) / 255)."""
+    _fields_ = [("obs", _fp), ("obs2", _fp), ("act", _fp), ("rew", _fp), ("done", _fp), ("logp", _fp),
+                ("capacity", C.c_int64)]
+
+
 # every symbol include/dsact.h declares: (restype, argtypes)
 IPC_HANDLE_BYTES = 64   # DSACT_IPC_HANDLE_BYTES
 DP_MAX_RANKS = 8        # DSACT_DP_MAX_RANKS
@@ -130,6 +136,8 @@ SYMBOLS = {
     "dsact_cnn_replay_bind": (C.c_int, [C.c_void_p, C.POINTER(Replay)]),
     "dsact_cnn_replay_add": (C.c_int, [C.c_void_p] + [C.c_void_p] * 6 + [C.c_int64, C.c_int64, C.c_void_p]),
     "dsact_cnn_replay_sample": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.POINTER(Batch), C.c_void_p]),
+    "dsact_cnn_replay_bind_u8": (C.c_int, [C.c_void_p, C.POINTER(ReplayU8)]),
+    "dsact_cnn_replay_add_u8": (C.c_int, [C.c_void_p] + [C.c_void_p] * 6 + [C.c_int64, C.c_int64, C.c_void_p]),
     "dsact_cnn_seed": (C.c_int, [C.c_void_p, C.c_uint64]),
     "dsact_cnn_step": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_int64, C.c_void_p]),
     "dsact_cnn_grad_phase1": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.POINTER(Noise), C.c_void_p]),

@@ -98,7 +98,9 @@ struct dsact_cnn_handle {
   int64_t ga, gb;             // conv-backward ping-pong buffers (largest activation)
   int64_t r_obs, r_obs2, r_act, r_rew, r_done, r_logp, r_idx;   // gathered replay minibatch
   dsact_replay rb;
-  bool rb_bound = false;
+  dsact_replay_u8 rb8;     // the 8-bit image ring, when rb_u8
+  bool rb_bound = false, rb_u8 = false;
+  int64_t rb_capacity() const { return rb_u8 ? rb8.capacity : rb.capacity; }
   int64_t dev_rb_size = -1;
   int64_t total;
   float* Wp() const { return reinterpret_cast<float*>(buf.workspace); }
@@ -627,6 +629,19 @@ static int cnn_finish(dsact_cnn_handle* h, const Ctx& c) {
   return DSACT_OK;
 }
 
+// rows (ptr + i) % capacity of every column: `cols` = (destination, source, bytes per row)
+struct RingCol { void* dst; const void* src; int64_t w; };
+static int cnn_ring_copy(const RingCol (&cols)[6], int64_t capacity, int64_t n, int64_t ptr, cudaStream_t s) {
+  const int64_t first = (ptr + n <= capacity) ? n : capacity - ptr;
+  for (const RingCol& c : cols) {
+    char* dst = static_cast<char*>(c.dst);
+    const char* src = static_cast<const char*>(c.src);
+    CUDA_TRY(cudaMemcpyAsync(dst + ptr * c.w, src, first * c.w, cudaMemcpyDefault, s));
+    if (first < n) CUDA_TRY(cudaMemcpyAsync(dst, src + first * c.w, (n - first) * c.w, cudaMemcpyDefault, s));
+  }
+  return DSACT_OK;
+}
+
 #include "v1_step.cuh"
 
 extern "C" {
@@ -712,33 +727,58 @@ int dsact_cnn_replay_bind(dsact_cnn_handle* h, const dsact_replay* rb) {
   if (!rb->obs || !rb->obs2 || !rb->act || !rb->rew || !rb->done || !rb->logp || rb->capacity < 1) return fail(DSACT_EINVAL, "bad replay buffers");
   h->rb = *rb;
   h->rb_bound = true;
+  h->rb_u8 = false;
   h->dev_rb_size = -1;
   return DSACT_OK;
+}
+
+int dsact_cnn_replay_bind_u8(dsact_cnn_handle* h, const dsact_replay_u8* rb) {
+  if (!h || !rb) return fail(DSACT_EINVAL, "null argument");
+  if (h->cfg.n_conv == 0)
+    return fail(DSACT_EINVAL, "dsact_cnn_replay_bind_u8: the handle has no conv encoder (n_conv = 0); 8-bit rings hold images on "
+                              "the 1/255 grid, vector observations stay in the fp32 ring");
+  if (!rb->obs || !rb->obs2 || !rb->act || !rb->rew || !rb->done || !rb->logp || rb->capacity < 1) return fail(DSACT_EINVAL, "bad replay buffers");
+  h->rb8 = *rb;
+  h->rb_bound = true;
+  h->rb_u8 = true;
+  h->dev_rb_size = -1;
+  return DSACT_OK;
+}
+
+int dsact_cnn_replay_add_u8(dsact_cnn_handle* h, const uint8_t* obs, const uint8_t* obs2, const float* act, const float* rew,
+                            const float* done, const float* logp, int64_t n, int64_t ptr, void* stream) {
+  if (!h || !h->rb_bound) return fail(DSACT_ESTATE, "replay buffer not bound");
+  if (!h->rb_u8) return fail(DSACT_ESTATE, "dsact_cnn_replay_add_u8: the bound ring stores fp32 images; use dsact_cnn_replay_add");
+  if (n < 0 || n > h->rb8.capacity || ptr < 0 || ptr >= h->rb8.capacity) return fail(DSACT_EINVAL, "bad n/ptr");
+  if (n == 0) return DSACT_OK;
+  if (!obs || !obs2 || !act || !rew || !done || !logp) return fail(DSACT_EINVAL, "null staging pointer");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const int64_t O = (int64_t)h->cfg.channels * h->cfg.height * h->cfg.width, A = h->cfg.act_dim;
+  const int64_t f = sizeof(float);
+  const RingCol cols[6] = {{h->rb8.obs, obs, O}, {h->rb8.obs2, obs2, O}, {h->rb8.act, act, A * f},
+                           {h->rb8.rew, rew, f}, {h->rb8.done, done, f}, {h->rb8.logp, logp, f}};
+  return cnn_ring_copy(cols, h->rb8.capacity, n, ptr, (cudaStream_t)stream);
 }
 
 int dsact_cnn_replay_add(dsact_cnn_handle* h, const float* obs, const float* obs2, const float* act, const float* rew,
                          const float* done, const float* logp, int64_t n, int64_t ptr, void* stream) {
   if (!h || !h->rb_bound) return fail(DSACT_ESTATE, "replay buffer not bound");
+  if (h->rb_u8) return fail(DSACT_ESTATE, "dsact_cnn_replay_add: the bound ring stores 8-bit images; use dsact_cnn_replay_add_u8");
   if (n < 0 || n > h->rb.capacity || ptr < 0 || ptr >= h->rb.capacity) return fail(DSACT_EINVAL, "bad n/ptr");
   if (n == 0) return DSACT_OK;
   if (!obs || !obs2 || !act || !rew || !done || !logp) return fail(DSACT_EINVAL, "null staging pointer");
   CUDA_TRY(cudaSetDevice(h->device));
-  const int64_t first = (ptr + n <= h->rb.capacity) ? n : h->rb.capacity - ptr;
   const int64_t O = (int64_t)h->cfg.channels * h->cfg.height * h->cfg.width, A = h->cfg.act_dim;
-  struct { float* dst; const float* src; int64_t w; } cols[6] = {
-      {h->rb.obs, obs, O}, {h->rb.obs2, obs2, O}, {h->rb.act, act, A}, {h->rb.rew, rew, 1}, {h->rb.done, done, 1}, {h->rb.logp, logp, 1}};
-  for (auto& c : cols) {
-    CUDA_TRY(cudaMemcpyAsync(c.dst + ptr * c.w, c.src, first * c.w * sizeof(float), cudaMemcpyDefault, (cudaStream_t)stream));
-    if (first < n)
-      CUDA_TRY(cudaMemcpyAsync(c.dst, c.src + first * c.w, (n - first) * c.w * sizeof(float), cudaMemcpyDefault, (cudaStream_t)stream));
-  }
-  return DSACT_OK;
+  const int64_t f = sizeof(float);
+  const RingCol cols[6] = {{h->rb.obs, obs, O * f}, {h->rb.obs2, obs2, O * f}, {h->rb.act, act, A * f},
+                           {h->rb.rew, rew, f}, {h->rb.done, done, f}, {h->rb.logp, logp, f}};
+  return cnn_ring_copy(cols, h->rb.capacity, n, ptr, (cudaStream_t)stream);
 }
 
 int dsact_cnn_replay_sample(dsact_cnn_handle* h, int32_t batch, int64_t size, const int64_t* idx, dsact_batch* out, void* stream) {
   if (!h || !h->bound || !h->rb_bound) return fail(DSACT_ESTATE, "not bound");
   if (batch < 1 || batch > h->cfg.max_batch) return fail(DSACT_EINVAL, "batch outside [1, max_batch]");
-  if (size < 1 || size > h->rb.capacity) return fail(DSACT_EINVAL, "size %lld outside [1, capacity]", (long long)size);
+  if (size < 1 || size > h->rb_capacity()) return fail(DSACT_EINVAL, "size %lld outside [1, capacity]", (long long)size);
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
   if (h->dev_rb_size != size) { set_rb_size_kernel<<<1, 32, 0, s>>>(h->buf.state, size); CUDA_TRY(cudaGetLastError()); h->dev_rb_size = size; }
@@ -749,9 +789,17 @@ int dsact_cnn_replay_sample(dsact_cnn_handle* h, int32_t batch, int64_t size, co
   int64_t* draw = idx ? nullptr : reinterpret_cast<int64_t*>(W + h->r_idx);
   int blocks = (batch + 7) / 8; if (blocks > 8 * h->num_sms) blocks = 8 * h->num_sms;
   const ImgOut none{nullptr, 0, 1, 0};
-  launch_k(gather_kernel, blocks, 256, 0, c, (const float*)h->rb.obs, (const float*)h->rb.obs2, (const float*)h->rb.act, (const float*)h->rb.rew,
-           (const float*)h->rb.done, (const float*)h->rb.logp, idx, W + h->r_obs, W + h->r_obs2, W + h->r_act, W + h->r_rew, W + h->r_done,
-           W + h->r_logp, (int)batch, O, A, none, none, none, draw, (unsigned long long)h->seed, (const float*)h->buf.state, 1);
+  if (h->rb_u8) {
+    const int wpb = GATHER_U8_THREADS / 32;
+    int b8 = (batch + wpb - 1) / wpb; if (b8 > 32 * h->num_sms) b8 = 32 * h->num_sms;
+    launch_k(gather_u8_kernel, b8, GATHER_U8_THREADS, 0, c, (const uint8_t*)h->rb8.obs, (const uint8_t*)h->rb8.obs2, (const float*)h->rb8.act,
+             (const float*)h->rb8.rew, (const float*)h->rb8.done, (const float*)h->rb8.logp, idx, W + h->r_obs, W + h->r_obs2, W + h->r_act,
+             W + h->r_rew, W + h->r_done, W + h->r_logp, (int)batch, O, A, draw, (unsigned long long)h->seed, (const float*)h->buf.state);
+  } else {
+    launch_k(gather_kernel, blocks, 256, 0, c, (const float*)h->rb.obs, (const float*)h->rb.obs2, (const float*)h->rb.act, (const float*)h->rb.rew,
+             (const float*)h->rb.done, (const float*)h->rb.logp, idx, W + h->r_obs, W + h->r_obs2, W + h->r_act, W + h->r_rew, W + h->r_done,
+             W + h->r_logp, (int)batch, O, A, none, none, none, draw, (unsigned long long)h->seed, (const float*)h->buf.state, 1);
+  }
   c.done();
   if (!idx) { launch_k(rng_advance_kernel, 1, 32, 0, c, h->buf.state); c.done(); }
   if (c.err != cudaSuccess) return fail(DSACT_ECUDA, "kernel launch failed: %s", cudaGetErrorString(c.err));

@@ -17,6 +17,7 @@
 #include "tc_host.cuh"
 #include "chain_tc.cuh"
 #include "dp_peer.cuh"
+#include "replay_u8.cuh"
 
 using namespace dsact;
 

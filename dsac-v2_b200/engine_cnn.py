@@ -10,7 +10,7 @@ from typing import Dict, Optional, Sequence
 import torch
 
 from . import _lib
-from ._lib import Batch, Buffers, CnnConfig, Layout, Noise, Replay, check
+from ._lib import Batch, Buffers, CnnConfig, Layout, Noise, Replay, ReplayU8, check
 from .engine import STAT_KEYS
 
 
@@ -220,22 +220,33 @@ class CnnEngine:
     def obs_elems(self) -> int:
         return self.cfg.channels * self.cfg.height * self.cfg.width
 
-    def bind_replay(self, capacity: int):
+    def bind_replay(self, capacity: int, obs_dtype: torch.dtype = torch.float32):
+        """Allocate and bind the device ring.  obs_dtype=torch.uint8 stores every image pixel as its code k (the pixel is
+        float32(k) / 255, decoded by the gather), a quarter of the fp32 ring's image bytes; it needs a conv encoder."""
+        if obs_dtype not in (torch.float32, torch.uint8):
+            raise ValueError(f"obs_dtype must be torch.float32 or torch.uint8, not {obs_dtype}")
         O, A = self.obs_elems, self.cfg.act_dim
         with torch.cuda.device(self.device):
-            z = lambda *s: torch.zeros(*s, dtype=torch.float32, device=self.device)
-            self.replay = dict(obs=z(capacity, O), obs2=z(capacity, O), act=z(capacity, A), rew=z(capacity), done=z(capacity), logp=z(capacity))
-            r = self.replay
-            rb = Replay(r["obs"].data_ptr(), r["obs2"].data_ptr(), r["act"].data_ptr(), r["rew"].data_ptr(), r["done"].data_ptr(),
-                        r["logp"].data_ptr(), int(capacity))
-            check(self.lib.dsact_cnn_replay_bind(self.h, C.byref(rb)))
+            z = lambda *s, dtype=torch.float32: torch.zeros(*s, dtype=dtype, device=self.device)
+            r = dict(obs=z(capacity, O, dtype=obs_dtype), obs2=z(capacity, O, dtype=obs_dtype), act=z(capacity, A), rew=z(capacity),
+                     done=z(capacity), logp=z(capacity))
+            ptrs = (r["obs"].data_ptr(), r["obs2"].data_ptr(), r["act"].data_ptr(), r["rew"].data_ptr(), r["done"].data_ptr(),
+                    r["logp"].data_ptr(), int(capacity))
+            if obs_dtype == torch.uint8:
+                check(self.lib.dsact_cnn_replay_bind_u8(self.h, C.byref(ReplayU8(*ptrs))))
+            else:
+                check(self.lib.dsact_cnn_replay_bind(self.h, C.byref(Replay(*ptrs))))
+        self.replay = r
         self.capacity = int(capacity)
 
     def replay_add(self, staging: Dict[str, torch.Tensor], n: int, ptr: int):
+        """Copy n staged rows into ring rows (ptr + i) % capacity.  uint8 obs / obs2 staging goes to an 8-bit ring, fp32
+        staging to an fp32 ring; the library refuses the other pairings."""
         s = staging
+        add = self.lib.dsact_cnn_replay_add_u8 if s["obs"].dtype == torch.uint8 else self.lib.dsact_cnn_replay_add
         with torch.cuda.device(self.device):
-            check(self.lib.dsact_cnn_replay_add(self.h, s["obs"].data_ptr(), s["obs2"].data_ptr(), s["act"].data_ptr(), s["rew"].data_ptr(),
-                                                s["done"].data_ptr(), s["logp"].data_ptr(), int(n), int(ptr), self._stream()))
+            check(add(self.h, s["obs"].data_ptr(), s["obs2"].data_ptr(), s["act"].data_ptr(), s["rew"].data_ptr(),
+                      s["done"].data_ptr(), s["logp"].data_ptr(), int(n), int(ptr), self._stream()))
 
     def replay_sample(self, batch: int, size: int, idx: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         out = Batch()
@@ -259,6 +270,13 @@ class CnnEngine:
     def seed(self, seed: int):
         self._seed = int(seed) & (2 ** 64 - 1)
         check(self.lib.dsact_cnn_seed(self.h, self._seed))
+
+    def set_carry(self, mean_std1=-1.0, mean_std2=-1.0, adam_steps_q=0, adam_steps_pi=0):
+        """Overwrite the carried scalars (mean_std EMA pair, Adam step counters), as `Engine.set_carry`: the drop-in's
+        load_full_state_dict restores them through this."""
+        with torch.cuda.device(self.device):
+            check(self.lib.dsact_cnn_set_carry(self.h, float(mean_std1), float(mean_std2), int(adam_steps_q), int(adam_steps_pi),
+                                               self._stream()))
 
     def read_stats_async(self, global_batch: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         out = self._stats_host if out is None else out

@@ -283,6 +283,26 @@ int dsact_cnn_replay_bind(dsact_cnn_handle *h, const dsact_replay *rb);
 int dsact_cnn_replay_add(dsact_cnn_handle *h, const float *obs, const float *obs2, const float *act, const float *rew,
                          const float *done, const float *logp, int64_t n, int64_t ptr, void *stream);
 int dsact_cnn_replay_sample(dsact_cnn_handle *h, int32_t batch, int64_t size, const int64_t *idx, dsact_batch *out, void *stream);
+/* The same ring with 8-bit images: obs / obs2 rows hold one uint8 code k per pixel, the pixel being float32(k) / 255.0f
+ * (IEEE correctly-rounded division).  That is exact for observations on the 1/255 grid, such as the reference's
+ * gym_carracingraw (rgb / 255, env_gym/gym_carracingraw_data.py:66-69), and takes a quarter of the fp32 ring's image bytes.
+ * Callers encode k = rint(x * 255) and accept a pixel only if the decoded value equals x bit for bit; values off the
+ * grid (e.g. gym_carracing's gray / 128 - 1) have no code and belong in the fp32 ring.  act / rew / done / logp stay fp32.
+ *  bind_u8: a handle without a conv encoder (n_conv = 0: vector observations) gets DSACT_EINVAL.  Binding either kind
+ *           replaces the ring bound before;
+ *  add_u8:  dsact_cnn_replay_add's rows (ptr + i) % capacity with uint8 obs / obs2 staging.  On an fp32 ring it returns
+ *           DSACT_ESTATE, and so does dsact_cnn_replay_add on an 8-bit ring;
+ *  dsact_cnn_replay_sample gathers from whichever kind was bound last and decodes into the same fp32 minibatch arena.
+ *           With idx = NULL it draws the same indices as on an fp32 ring (same seed and counter), so the two kinds of ring
+ *           holding the same transitions return identical minibatches. */
+typedef struct dsact_replay_u8 {
+  uint8_t *obs, *obs2;                         /* [capacity, O] codes */
+  float *act, *rew, *done, *logp;              /* [capacity, A], 3x [capacity] */
+  int64_t capacity;
+} dsact_replay_u8;
+int dsact_cnn_replay_bind_u8(dsact_cnn_handle *h, const dsact_replay_u8 *rb);
+int dsact_cnn_replay_add_u8(dsact_cnn_handle *h, const uint8_t *obs, const uint8_t *obs2, const float *act, const float *rew,
+                            const float *done, const float *logp, int64_t n, int64_t ptr, void *stream);
 
 /* introspection for tests/bench: number of kernel launches (graph nodes included)
  * submitted by this handle so far, and by the most recent entry-point call */
